@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- LR event-frames/sec of the ESR hot path on B200 (BASELINE.json metric), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg3|cfg4] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg3|cfg4] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one batch of B sequences x L LR event frames taken from raw events to redistributed SR events:
@@ -22,6 +22,9 @@ the workload on its own shard (weak scaling) and the time is the max over ranks.
 exchange of the path: the NCCL all-reduce of the flat gradient, captured with the iteration in one CUDA graph.
 `--impl reference` times the CPU restatement of the same path on the host cores (rank 0 only): the oracle port of the
 network plus the reference's OWN compiled Cython redistribution (oracle/_ref) when it was built.
+`--dump-outputs DIR` writes what the last timed step of the headline workload returned (rank 0): sr_counts.npy and
+events.npy, float32, at most 64 MB together (a fixed seeded sample beyond that).  Inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -36,6 +39,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree bench.py runs from may be read-only: nothing is cached in it
 
 WORKLOADS = {
     # BASELINE.json configs[1]: 2x SR, seq_len=8, LR 128x128, batch=8 per GPU
@@ -48,6 +52,7 @@ WORKLOADS = {
 EVENTS_PER_FRAME = 2048          # config/train_ours_enfssyn.yml:9 WINDOW
 FLOP_PER_HR_PIXEL = 184.7e3      # SURVEY.md 8d
 PARITY_TOL = 1e-3                # BASELINE.json north_star: within 1e-3 rel on fp32 count tensors
+DUMP_BYTES = 60 << 20            # --dump-outputs: payload of all .npy files together (keeps the directory under 64 MB)
 
 
 def synth_events(B, L, lr, seed):
@@ -85,6 +90,21 @@ def synth_sr_bias(B, L, hr, seed):
     `model output + Poisson(0.3)` synthetic counts (BASELINE.md 3) to do representative work."""
     g = torch.Generator().manual_seed(seed + 17)
     return torch.poisson(torch.full(((L - 2) * B, 2, hr[0], hr[1]), 0.3), generator=g)
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Writes each tensor of `arrays` as out_dir/<name>.npy in float32.  When all of them together exceed `budget`, each one is
+    replaced by a fixed sample of its flattened elements (seed 0, ascending index, a share of the budget proportional to its
+    size): the same shapes give the same indices, so two builds run with the same arguments compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() for t in arrays.values()) * 4
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if total > budget:
+            k = t.numel() * budget // total
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), k))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 class ClockSampler(threading.Thread):
@@ -567,18 +587,18 @@ def run_workload(args, name, dev, rank, world, dist, steps, warmup, main):
         torch.cuda.synchronize()
 
     def timed(fn, k):
-        """per-step CUDA-event timing with an (untimed) L2 flush between steps; returns total ms"""
-        tot = 0.0
+        """per-step CUDA-event timing with an (untimed) L2 flush between steps; returns (total ms, what the last step returned)"""
+        tot, out = 0.0, None
         for _ in range(k):
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             torch.cuda.synchronize()
             e0.record()
-            fn()
+            out = fn()
             e1.record()
             torch.cuda.synchronize()
             tot += e0.elapsed_time(e1)
-        return tot
+        return tot, out
 
     dev_step = lambda: pipe.run_device(d_xs, d_ys, d_ps, d_off, EVENTS_PER_FRAME)
     host_step = lambda: pipe.run_host(h_xs, h_ys, h_ps, h_off, EVENTS_PER_FRAME)
@@ -595,10 +615,13 @@ def run_workload(args, name, dev, rank, world, dist, steps, warmup, main):
         sampler.start()
     barrier()
     l0 = _lib.lib().esr_launch_count()
-    ms_dev = timed(dev_step, steps)
+    ms_dev, last = timed(dev_step, steps)
     launches = _lib.lib().esr_launch_count() - l0 + steps * pipe.graph_launches
+    if main and rank == 0 and args.dump_outputs:                      # before the next step overwrites the graph's output buffers
+        dump_outputs(args.dump_outputs, {"sr_counts": last[0], "events": last[1]})
+    del last
     barrier()
-    ms_e2e_sync = timed(host_step, steps) if main else 0.0            # one batch at a time (latency view)
+    ms_e2e_sync = timed(host_step, steps)[0] if main else 0.0         # one batch at a time (latency view)
     barrier()
 
     # throughput view of the same end-to-end path: submit(i+1) is issued before finish(i), so the GPU runs batch i+1's network while
@@ -827,7 +850,11 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the training-iteration measurement (the `train` key)")
     ap.add_argument("--no-parity", action="store_true", help="skip the un-timed oracle check of the measured plan")
     ap.add_argument("--no-extra", action="store_true", help="skip the other configs (cfg3 / cfg4) and the cfg5 sweep")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (SR count tensors, event lists) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE line (the JSON): anything a library prints there (NCCL's version banner at N > 1) goes to stderr
     sys.stdout.flush()
     json_fd = os.dup(1)

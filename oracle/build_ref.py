@@ -60,8 +60,9 @@ def build(force=False):
 
 
 def import_ref_modules():
-    """(cnt2event, event_redistribute) reference modules, or (None, None) if not built."""
-    if not build():
+    """(cnt2event, event_redistribute) reference modules, or (None, None) if not built.  Builds nothing: its caller
+    (bench.py) may run from a read-only tree."""
+    if not all(os.path.exists(p) for p in built_paths()):
         return None, None
     import importlib.util
     mods = []

@@ -9,10 +9,12 @@ Each function mirrors the reference call it restates:
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
+_SRC = os.path.join(_HERE, "esr_oracle.c")
 _SO = os.path.join(_HERE, "_build", "libesr_oracle.so")
 _lib = None
 
@@ -21,19 +23,25 @@ _f64p = ctypes.POINTER(ctypes.c_double)
 _i64p = ctypes.POINTER(ctypes.c_int64)
 
 
-def build(force=False):
-    src = os.path.join(_HERE, "esr_oracle.c")
-    if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        os.makedirs(os.path.dirname(_SO), exist_ok=True)
-        subprocess.check_call(["gcc", "-O2", "-ffp-contract=off", "-fPIC", "-shared", src, "-o", _SO, "-lm"])
-    return _SO
+def _stale(so):
+    return not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(_SRC)
+
+
+def build(force=False, so=_SO):
+    if force or _stale(so):
+        os.makedirs(os.path.dirname(so), exist_ok=True)
+        subprocess.check_call(["gcc", "-O2", "-ffp-contract=off", "-fPIC", "-shared", _SRC, "-o", so, "-lm"])
+    return so
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        _lib = ctypes.CDLL(_SO)
+        if not _stale(_SO):
+            _lib = ctypes.CDLL(_SO)
+        else:                       # not built, or older than its source: compile outside the tree, which may be read-only
+            with tempfile.TemporaryDirectory() as d:
+                _lib = ctypes.CDLL(build(so=os.path.join(d, "libesr_oracle.so")))
         _lib.oracle_total_events.restype = ctypes.c_int64
     return _lib
 
